@@ -1,6 +1,6 @@
 """Benchmark of the StreamYOLO hot path: frame-pairs/s of forward+loss (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model l] [--batch 8]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--model l] [--batch 8] [--dump-outputs DIR]
 
 One process per GPU (torchrun sets RANK/LOCAL_RANK/WORLD_SIZE for N > 1).  A "step" is one pass of
 the hot path -- DFPPAFPN (CSPDarknet + PAFPN on both frames, DFP fusion) + TALHead + SimOTA/TAL loss,
@@ -399,6 +399,8 @@ def run_reference(args, rank):
     pairs = 2
     steps, warmup = max(1, args.steps), max(0, args.warmup)
     v, sec = cpu_oracle_run(args.model, pairs, steps, warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: LAST_ORACLE_LOSS[k] for k in LOSS_KEYS})
     line = {"impl": "reference", "metric": "frame-pairs/sec StreamYOLO-%s 600x960 fwd+loss" % args.model,
             "value": round(v, 4), "unit": "pairs/s", "n_gpus": args.gpus, "steps": steps, "warmup": warmup,
             "ms_per_step": round(sec * 1e3, 2), "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
@@ -434,6 +436,15 @@ def emit(text):
     print(text, file=out, flush=True)
 
 
+def dump_outputs(path, outputs):
+    """--dump-outputs: what the timed path returned in its last step, one float32 DIR/<name>.npy per output, so that two
+    builds run with the same arguments (hence the same seeded inputs) can be compared output for output."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, v in outputs.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(v, dtype=np.float32))
+
+
 def main():
     guard_stdout()
     ap = argparse.ArgumentParser()
@@ -447,7 +458,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-train", action="store_true", help="skip the training-step measurements (configs 2-4)")
     ap.add_argument("--no-extras", action="store_true", help="skip the sustained run, eval / on_pipe modes and the conv-family timing")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the six loss outputs of the last timed step as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     from streamyolo_b200 import dist as sydist
@@ -527,6 +542,8 @@ def main():
         clocks = sampler.stop()
         ms_step = ms_total / args.steps
         value = world * B / (ms_step * 1e-3)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, dict(zip(LOSS_KEYS, loss_vec.cpu().tolist())))
 
         # ---------------- end-to-end: host inputs, H2D every step (double buffered), D2H of the result
         copy_stream = torch.cuda.Stream()

@@ -1,12 +1,12 @@
 """Generate tests/golden/*.npz FROM THE UNMODIFIED REFERENCE (test infrastructure).
 
-Runs only in the build container, where /root/reference is mounted:
+Needs a checkout of the original StreamYOLO project:
 
-    python oracle/make_golden.py            # writes tests/golden/<case>.npz
+    python oracle/make_golden.py REFERENCE_DIR [case ...]    # writes tests/golden/<case>.npz
 
-It imports /root/reference/exps/model/{yolox,dfp_pafpn,darknet,tal_head}.py untouched, on
-top of the yolox==0.3.0 stand-in in oracle/ref_shim (the real package is absent and
-un-installable here), loads the deterministic synthetic state_dict / frames / labels of
+It imports REFERENCE_DIR/exps/model/{yolox,dfp_pafpn,darknet,tal_head}.py untouched, on
+top of the yolox==0.3.0 stand-in in oracle/ref_shim (the real package is not a
+dependency of this project), loads the deterministic synthetic state_dict / frames / labels of
 ``streamyolo_b200.synth``, and records what the reference computes on CPU fp32:
 
   * train forward (model.train(), head.use_l1=True, BN eps 1e-3 / momentum 0.03 as
@@ -18,7 +18,9 @@ un-installable here), loads the deterministic synthetic state_dict / frames / la
     a sub-sample of the decoded [B, A, 13] output plus checksums;
   * on_pipe: first call and a buffered second call.
 
-Nothing on the GPU box reads /root/reference; the committed .npz files are the pin.
+Importing this module (the tests take CASES from it) leaves sys.path alone apart from the
+repository root; only the script run puts the original project on it.  Nothing else reads the
+original project: the committed .npz files are the pin.
 """
 import os
 import sys
@@ -29,8 +31,6 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 sys.path.insert(0, ROOT)
-sys.path.insert(0, os.path.join(HERE, "ref_shim"))
-sys.path.insert(0, "/root/reference")
 
 from streamyolo_b200 import synth  # noqa: E402
 
@@ -182,8 +182,12 @@ def shapes_fixture():
 
 
 if __name__ == "__main__":
+    if len(sys.argv) < 2 or not os.path.isdir(os.path.join(sys.argv[1], "exps", "model")):
+        sys.exit("usage: python oracle/make_golden.py REFERENCE_DIR [case ...]  (REFERENCE_DIR: a StreamYOLO checkout)")
+    sys.path.insert(0, os.path.join(HERE, "ref_shim"))
+    sys.path.insert(0, os.path.abspath(sys.argv[1]))
     torch.set_num_threads(os.cpu_count())
-    only = sys.argv[1:]
+    only = sys.argv[2:]
     if not only or "shapes" in only:
         shapes_fixture()
     for n, c in CASES.items():
